@@ -13,6 +13,7 @@ Excluded like SURVEY 8d says: CLIP losses, PNG dumps, the Adan update.  Syntheti
   python bench.py --gpus 1 --steps 10 --warmup 3            # one JSON line
   torchrun ... bench.py --gpus N ...                        # one rank per GPU, weak scaling (one view per GPU per step)
   python bench.py --impl reference ...                      # the reference algorithm on the host CPU cores (oracle port)
+  python bench.py ... --dump-outputs DIR                    # also write what the last timed step computed to DIR/<name>.npy
 """
 import argparse
 import importlib
@@ -21,6 +22,7 @@ import math
 import os
 import subprocess
 import sys
+import tempfile
 import threading
 import time
 
@@ -136,6 +138,16 @@ def regulariser_loss(out, opt):
     return loss
 
 
+def dump_outputs(path, out, loss, model):
+    """What the last timed step handed its caller: the render outputs, the total loss, and the gradients it left on the NeRF
+    parameters (SDS + regularisers, summed over ranks), one float32 .npy per array (about 47 MiB in all)."""
+    os.makedirs(path, exist_ok=True)
+    arrays = dict(out, loss=loss, grad_encoder=model.encoder.params.grad)
+    arrays.update({"grad_sigma_net." + n: p.grad for n, p in model.sigma_net.named_parameters()})
+    for name, t in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), t.detach().float().cpu().numpy())
+
+
 def run_ours(args):
     par = importlib.import_module("make-it-3d_b200.parallel")
     field_ops = importlib.import_module("make-it-3d_b200.nerf.field_ops")
@@ -206,6 +218,8 @@ def run_ours(args):
             marks.append(_ev())
         loss = loss + regulariser_loss(out, opt)
         loss.backward()
+        state["out"] = {k: v.detach() for k, v in out.items()}
+        state["loss"] = loss.detach()
         if marks is not None:
             marks.append(_ev())
         reducer()
@@ -309,6 +323,8 @@ def run_ours(args):
     i_first = state["i"]
     ms = timed(args.steps, False, args.warmup)
     m_timed = m_log[[(i_first + k) % m_log.numel() for k in range(args.steps)]].cpu().numpy().astype(np.int64)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, state["out"], state["loss"], model)
     # ---- per-kernel live timing of the dominant kernels (CUDA events on the launching stream) ----
     import ctypes as C
     L = importlib.import_module("make-it-3d_b200._lib")
@@ -332,13 +348,14 @@ def run_ours(args):
             step(args.warmup + s, False)
         torch.cuda.synchronize()
     gemm_ms, gemm_n = C.c_float(0), C.c_int(0)
-    dump_path = os.path.join(ROOT, "gpurun_out", f"sd_launches_rank{rank}.txt")
-    os.makedirs(os.path.dirname(dump_path), exist_ok=True)
-    # one line per timed launch: M N K block_n splits conv batch epi ms
-    L.check(L.lib().mi3d_sd_profile_dump(guidance.engine.h, C.c_int(0), C.byref(gemm_ms), C.byref(gemm_n), dump_path.encode()), "sd_profile_dump")
+    # one line per timed launch: M N K block_n splits conv batch epi ms (in a scratch directory: the tree may be read-only)
+    with tempfile.TemporaryDirectory() as tmp:
+        dump_path = os.path.join(tmp, "sd_launches.txt")
+        L.check(L.lib().mi3d_sd_profile_dump(guidance.engine.h, C.c_int(0), C.byref(gemm_ms), C.byref(gemm_n), dump_path.encode()), "sd_profile_dump")
+        launches = open(dump_path).read().splitlines()
     tile_flops = attn_flops = attn_ms = 0.0
     attn_n = 0
-    for ln in open(dump_path):
+    for ln in launches:
         f = ln.split()
         Mm, Nn, Kk, conv, batch, ms_l = int(f[0]), int(f[1]), int(f[2]), int(f[5]), int(f[6]), float(f[8])
         if conv == 2:
@@ -517,7 +534,13 @@ def main():
     ap.add_argument("--launch-list", action="store_true",
                     help="profiling aid: warm up, run --steps steps of the same step function and exit (use under "
                          "`ncu --metrics gpu__time_duration.sum`; numbers printed under a profiler are never bench values)")
+    ap.add_argument("--dump-outputs", default=None, metavar="DIR",
+                    help="after the timed steps, write what the last one computed (render outputs, loss, parameter gradients) to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl == "reference" or args.timeline or args.launch_list):
+        ap.error("--dump-outputs writes the outputs of the timed steps: not with --impl reference, --timeline or --launch-list")
     if args.impl == "reference":
         run_reference(args)
     else:

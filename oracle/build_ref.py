@@ -4,7 +4,8 @@
 copied into the repo.  Differences from the reference's own recipe (raymarching/backend.py:6-12): -std=c++17 instead of
 c++14 (torch >= 2.1 headers need it) and an explicit -gencode for sm_100a (the reference passes no arch at all).
 
-Used by tests/test_ref_parity_gpu.py (-m gpu) to pin the CPU oracle and the CUDA path against the real reference kernels.
+Used by tests/golden/make_golden_ref_raymarching.py to record the real reference kernels' outputs, against which
+tests/test_ref_parity_gpu.py and tests/test_backend_dropin_gpu.py pin the CPU oracle and the CUDA path.
 """
 import os
 import sys

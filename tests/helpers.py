@@ -33,6 +33,15 @@ def camera_rays(HW, radius=1.25, theta=80.0, phi=170.0, fov=20.0):
     return ro.numpy(), rd.numpy(), sc.numpy()
 
 
+def march_rows(ro, rd, bits, nears, fars, noises, max_steps=512):
+    """The oracle's training march (ray-id order, bit-identical to ours) in N * max_steps caller-allocated rows, the way the
+    reference wrapper allocates them: (deltas [N * max_steps, 2], rays [N, 3], number of samples)."""
+    _, _, dl, rays, m = orm.march_rays_train(ro, rd, 1.0, bits, 1, 128, nears, fars, noises, 0.0, max_steps, align=-1)
+    deltas = np.zeros((ro.shape[0] * max_steps, 2), np.float32)
+    deltas[:m] = dl[:m]
+    return deltas, rays, m
+
+
 def field_from_golden(g):
     """oracle FieldRef holding the fixture's parameters."""
     f = fr.FieldRef(bound=1.0, blob_density=5.0, blob_radius=0.1, seed=0)
