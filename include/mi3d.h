@@ -466,6 +466,23 @@ int mi3d_sd_graph_replays(mi3d_sd_t h);
 /* debug tap: device pointer + size of a named intermediate ("unet.mid", "vae.grad_in", ...) */
 int mi3d_sd_debug_tensor(mi3d_sd_t h, const char* name, void** ptr, size_t* bytes);
 
+/* ------------------------------------------------------------------------------------------------------
+ * B4: refine-stage point renderer  (replaces pytorch3d rasterize_points + compositing.alpha_composite as called by
+ *     render_point, nerf/refine_utils.py:306-333)
+ * ------------------------------------------------------------------------------------------------------
+ * Square S x S image.  pts_ndc [P,3]: NDC x, y (pixel (row i, column j) has centre (-1 + (2 (S-1-j) + 1) / S, same for i)) and
+ * camera depth z; points with z < 0 or a non-finite coordinate are skipped.  A point is a candidate of a pixel when its squared
+ * NDC distance d <= radius^2; each pixel keeps the K (1..16) candidates of smallest (z, point index), ascending:
+ * idx [S,S,K] int32 (-1 = empty), dists [S,S,K] fp32 (d; -1 = empty).  With a_k = 1 - sqrt(clamp(0.1 d_k / radius^2, 1e-3, 1)),
+ * T_0 = 1, T_k+1 = T_k (1 - a_k):  out [C,S,S] = sum_k T_k a_k feats[idx_k].  Background is 0.
+ * workspace: mi3d_point_render_workspace_bytes(P, S, K, radius) bytes (tile lists; 0 = bad arguments).
+ * backward: g_feats [P,C] (overwritten) from g_out [C,S,S] and the forward's idx / dists; deterministic, no atomics. */
+size_t mi3d_point_render_workspace_bytes(uint32_t P, uint32_t S, uint32_t K, float radius);
+int mi3d_point_render_forward(const float* pts_ndc, const float* feats, uint32_t P, uint32_t C, uint32_t S, uint32_t K, float radius,
+                              int* idx, float* dists, float* out, void* workspace, size_t workspace_bytes, mi3d_stream_t stream);
+int mi3d_point_render_backward(const float* g_out, const float* pts_ndc, const int* idx, const float* dists, uint32_t P, uint32_t C,
+                               uint32_t S, uint32_t K, float radius, float* g_feats, mi3d_stream_t stream);
+
 /* unit-test entry for the hand-written kind::tf32 tiles of the field kernels (3-term split, K-major / MN-major operands):
  * mode 0: d[128,N] = a[128,K] . b[N,K]^T ; mode 1: d = a[K,128]^T . b[K,N] ; mode 2: d = a[128,K] . b[K,N].  fp32 in/out. */
 int mi3d_tf32_tile_test(const float* a, const float* b, float* d, int N, int K, int mode, mi3d_stream_t stream);

@@ -105,6 +105,7 @@ SYMBOLS = [
     "mi3d_sd_workspace_bytes", "mi3d_sd_create", "mi3d_sd_destroy", "mi3d_sd_num_params", "mi3d_sd_param_name", "mi3d_sd_param_numel",
     "mi3d_sd_param_shape", "mi3d_sd_load_param", "mi3d_sd_encode", "mi3d_sd_encode_backward", "mi3d_sd_unet_sds", "mi3d_sd_debug_tensor", "mi3d_sd_profile",
     "mi3d_sd_profile_dump", "mi3d_sd_set_graph_replay", "mi3d_sd_graph_replays", "mi3d_sd_ddim_step", "mi3d_sd_decode",
+    "mi3d_point_render_workspace_bytes", "mi3d_point_render_forward", "mi3d_point_render_backward",
 ]
 
 
@@ -132,6 +133,7 @@ def lib():
         _lib.mi3d_render_workspace_bytes.restype = C.c_size_t
         _lib.mi3d_sumsq_workspace_bytes.restype = C.c_size_t
         _lib.mi3d_render_eval_workspace_bytes.restype = C.c_size_t
+        _lib.mi3d_point_render_workspace_bytes.restype = C.c_size_t
         for name in ("mi3d_sd_workspace_bytes", "mi3d_sd_weight_bytes"):
             if hasattr(_lib, name):
                 getattr(_lib, name).restype = C.c_size_t
